@@ -1,9 +1,10 @@
 """Benchmark of the RoboSat segmentation hot path on B200 (BASELINE.json).
 
-    python bench.py [--gpus N --steps K --warmup W] [--impl reference]
+    python bench.py [--gpus N --steps K --warmup W] [--impl reference] [--dump-outputs DIR]
     torchrun ... bench.py --gpus N ...           (one rank per GPU, NCCL)
 
-Prints ONE JSON line (rank 0).
+Prints ONE JSON line (rank 0). --dump-outputs DIR writes what the last timed step of each precision returned (rank 0) as
+DIR/<precision>_logits.npy and DIR/<precision>_bins.npy, so that two builds can be compared output for output.
 
 Headline = BASELINE.json configs[1] (`rs predict`: ResNet50-UNet, 2 classes, synthetic 3x512x512 tiles, batch 32 per GPU) in the
 STRICT precision -- the mode whose outputs meet the parity contract (logits 1e-3 rel, argmax identical up to the fp32 noise
@@ -15,8 +16,7 @@ max-pools, softmax/crop/quantise head).
     roofline   executed tensor FLOP/s of the dominant convolution instantiation (timed alone -> against the BURST bf16 peak
                of MEASURED_PEAKS.json; the sustained fraction and the whole-step rate are printed beside it)
     fast       the same three for the fast precision (single fp16 operands, logits ~2e-3): labelled secondary
-    sustained  (when K < 100) the same step timed for >= 1.5 s, i.e. at the board's power cap instead of a burst
-    cpu_baseline  the UNMODIFIED reference (baseline/_ref, torch CPU fp32) on a bounded sample of the workload (N=1 only)
+    cpu_baseline  the UNMODIFIED reference (oracle/_ref, torch CPU fp32) on a bounded sample of the workload (N=1 only)
 Other BASELINE configs, each a sub-record measured at the N the run was launched with:
     train      configs[2]: rs train step (2-class, Lovasz, 3x512x512, batch 16 per GPU) incl. the gradient all-reduce
     train_cfg5 configs[4]: 6-class, 3x1024x1024, batch 8 per GPU, data-parallel over N GPUs (ms in NCCL vs compute)
@@ -110,9 +110,9 @@ def host_threads():
 
 
 def cpu_reference_leg(steps, warmup, tiles_per_step, threads=None):
-    """The reference's own predict step on the CPU, through its public classes, unmodified (baseline/_ref):
+    """The reference's own predict step on the CPU, through its public classes, unmodified (oracle/_ref):
     `net = DataParallel(UNet(2)); outputs = net(images); probs = softmax(outputs, 1).data.cpu().numpy()` (predict.py:47-87).
-    Falls back to the oracle restatement (kind "port") only when baseline/_ref is not installed."""
+    Falls back to the oracle restatement (kind "port") only when oracle/_ref is not installed."""
     import torch
 
     from robosat_b200 import synth
@@ -274,7 +274,25 @@ def layer_profile(engine, x, reps=3):
     return rows
 
 
-def predict_leg(precision, sd, dev, rank, world, steps, warmup, dist, with_clocks, layers_out=None):
+DUMP_PIXELS = 1 << 20  # of the 8.4 M output pixels of a batch: 12 MB per precision instead of 96 MB
+
+
+def dump_outputs(out_dir, precision, logits, bins):
+    """Writes what one predict step hands its caller -- fp32 logits [N, C, H, W] and the uint8 foreground bins [N, H, W] --
+    at the same DUMP_PIXELS pixels, drawn once with a fixed seed: <precision>_logits.npy [DUMP_PIXELS, C] and
+    <precision>_bins.npy [DUMP_PIXELS], both float32."""
+    import numpy as np
+    import torch
+
+    n, c, h, w = logits.shape
+    pix = torch.randperm(n * h * w, generator=torch.Generator().manual_seed(0))[:DUMP_PIXELS].sort().values.to(logits.device)
+    os.makedirs(out_dir, exist_ok=True)
+    sampled = {"logits": logits.reshape(n, c, h * w)[pix // (h * w), :, pix % (h * w)], "bins": bins.reshape(-1)[pix]}
+    for name, t in sampled.items():
+        np.save(os.path.join(out_dir, "%s_%s.npy" % (precision, name)), t.float().cpu().numpy())
+
+
+def predict_leg(precision, sd, dev, rank, world, steps, warmup, dist, with_clocks, layers_out=None, dump_dir=None):
     import torch
 
     from robosat_b200 import synth
@@ -303,8 +321,8 @@ def predict_leg(precision, sd, dev, rank, world, steps, warmup, dist, with_clock
         barrier()
         return e0.elapsed_time(e1)
 
-    # nvidia-smi needs ~1 s to start reporting and samples every 100 ms: the sampler covers warm-up, the timed K steps and
-    # the sustained run that follows, all of them the same back-to-back step
+    # nvidia-smi needs ~1 s to start reporting and samples every 100 ms: the sampler covers warm-up and the timed K steps,
+    # all of them the same back-to-back step
     sampler = ClockSampler(dev.index)
     if rank == 0 and with_clocks:
         sampler.start()
@@ -313,13 +331,11 @@ def predict_leg(precision, sd, dev, rank, world, steps, warmup, dist, with_clock
         step(i)
     barrier()
     ms = timed(steps)
-    sustained_ms = sustained_steps = None
-    if steps < 100:
-        sustained_steps = max(100, int(1500.0 / max(ms / steps, 1e-3)))  # >= 1.5 s of back-to-back steps: the power-capped regime
-        sustained_ms = timed(sustained_steps)
     clocks = sampler.stop() if rank == 0 and with_clocks else None
     if clocks is not None:
-        clocks["window"] = "warm-up + the %d timed steps%s" % (steps, " + the sustained run" if sustained_steps else "")
+        clocks["window"] = "warm-up + the %d timed steps" % steps
+    if dump_dir and rank == 0:
+        dump_outputs(dump_dir, precision, pred.engine.logits, qbuf)
 
     # end to end through the host API: pinned host tiles in, uint8 bins out, copies inside the timed region
     host_batches = [synth.make_tiles_u8(BATCH, TILE, seed=200 + rank * 10 + i).pin_memory() for i in range(2)]
@@ -340,19 +356,15 @@ def predict_leg(precision, sd, dev, rank, world, steps, warmup, dist, with_clock
     e2e_ms = e2.elapsed_time(e3)
     wall_ms = (time.perf_counter() - t0) * 1e3
 
-    vals = [ms, e2e_ms, wall_ms, sustained_ms or 0.0]
+    vals = [ms, e2e_ms, wall_ms]
     if world > 1:
         t = torch.tensor(vals, device=dev, dtype=torch.float64)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         vals = t.tolist()
-    ms, e2e_ms, wall_ms, sustained_ms = vals
+    ms, e2e_ms, wall_ms = vals
 
     out = {"precision": precision, "ms": ms, "e2e_ms": e2e_ms, "wall_ms": wall_ms, "clocks": clocks, "launches": pred.num_launches(),
            "h2d": pred.h2d_bytes, "d2h": pred.d2h_bytes}
-    if sustained_steps:
-        out["sustained"] = {"steps": sustained_steps, "ms_per_step": sustained_ms / sustained_steps,
-                            "value": world * BATCH * sustained_steps / (sustained_ms / 1e3), "unit": "tiles/s",
-                            "note": ">= 1.5 s of back-to-back steps (board power cap) vs the %d-step burst of `value`" % steps}
     if rank == 0:
         pk = peaks()
         rows = layer_profile(pred.engine, inputs[0])
@@ -680,7 +692,10 @@ def main():
     ap.add_argument("--cfg4-tiles", type=int, default=0, help="tiles per GPU in the synthetic slippy-map directory (0: 2048 up to 2 GPUs, 512 beyond)")
     ap.add_argument("--tiles-per-step", type=int, default=0, help="(--impl reference) tiles per step instead of the automatic bounded sample")
     ap.add_argument("--layers-out", default=None, help="write the per-layer timing tables (JSON) here (_strict / _fast suffix)")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR", help="(--impl ours) write the outputs of the last timed step of each precision here (.npy)")
     args = ap.parse_args()
+    if args.impl == "reference" and args.dump_outputs:
+        ap.error("--dump-outputs writes the outputs of the timed predict path of --impl ours; --impl reference has none to write")
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -719,8 +734,8 @@ def main():
 
         sd = broadcast_state_dict(sd if rank == 0 else None, template=sd, device=dev)  # rank 0 is the only one whose copy is used
 
-    strict = predict_leg("strict", sd, dev, rank, world, args.steps, args.warmup, dist, True, args.layers_out)
-    fast = predict_leg("fast", sd, dev, rank, world, args.steps, args.warmup, dist, False, args.layers_out)
+    strict = predict_leg("strict", sd, dev, rank, world, args.steps, args.warmup, dist, True, args.layers_out, args.dump_outputs)
+    fast = predict_leg("fast", sd, dev, rank, world, args.steps, args.warmup, dist, False, args.layers_out, args.dump_outputs)
 
     extras = {}
     if not args.no_extras:
@@ -743,8 +758,6 @@ def main():
                  "e2e": {"value": tiles / (r["e2e_ms"] / 1e3), "unit": "tiles/s", "h2d_bytes_per_step": r["h2d"], "d2h_bytes_per_step": r["d2h"],
                          "wall_ms": r["wall_ms"], "api": "TilePredictor.submit/collect (pinned uint8 in, uint8 bins out)"},
                  "roofline": r.get("roofline")}
-            if "sustained" in r:
-                s["sustained"] = r["sustained"]
             return s
 
         s, f = summary(strict), summary(fast)
@@ -757,8 +770,6 @@ def main():
                 "fast": dict(f, precision="fast", dtype="f16 operands (1 MMA per K step), fp32 accumulate",
                              note="secondary: logits ~2e-3 rel, ~0.1 % argmax flips at near-ties -- does NOT meet the parity contract",
                              dense_equiv_tflops=f["value"] * FWD_GFLOP_DENSE / 1e3)}
-        if "sustained" in s:
-            line["sustained"] = s["sustained"]
         line.update(extras)
         if world == 1 and not args.no_extras:
             if not args.no_cpu_baseline:  # the CPU baseline is an N=1 figure (rank 0 only), ~10-30 s of CPU work
