@@ -280,8 +280,8 @@ def run_train_ops(eng, ops, x=None, dlogits=None):
             _, b, dy, y, dz, g_out = op
             pf = b.prefix
             g = dy.reshape(b.M, b.C).float()
-            if y is not None:
-                g = g * (y.reshape(b.M, b.C).float() > 0)
+            if y is not None:  # masked entries are +0, as autograd's threshold_backward writes them
+                g = torch.where(y.reshape(b.M, b.C).float() > 0, g, torch.zeros(()))
             zhat = (b.z.reshape(b.M, b.C).float() - b.mean) * b.invstd
             s0 = g.double().sum(0)
             s1 = (g * zhat).double().sum(0)
@@ -297,7 +297,7 @@ def run_train_ops(eng, ops, x=None, dlogits=None):
             if b2 is not None:
                 g = g + b2.float()
             if y is not None:
-                g = g * (y.float() > 0)
+                g = torch.where(y.float() > 0, g, torch.zeros(()))
             out.copy_(g.half())
         elif k == "maxpool":
             _, src, dst, n, h, w, c, kk, s, p = op
