@@ -381,6 +381,42 @@ int rsb_unpack_grads(const float* packed_grad, const int32_t* map4, float* grad,
 int rsb_unpack_grads_gather(const float* packed_grad, const int32_t* dst_idx, const int32_t* inv4, float* grad, int64_t n, float mul,
                             void* stream);
 
+/* Strict-precision training forward (the opt-in `strict` training plan): forward activations are fp16 (hi, lo) pairs in two
+ * planes `plane` elements apart (value = hi + lo, exact in fp32; hi = half(v), lo = half(v - hi)), as the split convolutions
+ * (rsb_conv_desc.split) read and write them. The backward keeps single fp16 operands and reads the hi planes.
+ *
+ * fp32 OIHW master weights -> split packed operand: dst[i] = hi, dst[plane + i] = lo of (sum of the map's sources) * scale, scale a
+ * power of two fixed per layer (the conv's acc_scale is its inverse). Every element whose scaled hi is not a finite fp16 adds one to
+ * *overflow (int32 on the device, never reset by the call): the weights have outgrown the layer's exponent. map4 / map1 as in
+ * rsb_pack_weights / rsb_pack_weights1 (the 1-index form: n and plane multiples of 8, map and dst 16-byte aligned). */
+int rsb_pack_weights_split(const float* src, const int32_t* map4, void* dst, int64_t plane, int64_t n, float scale, int32_t* overflow,
+                           void* stream);
+int rsb_pack_weights1_split(const float* src, const int32_t* map1, void* dst, int64_t plane, int64_t n, float scale, int32_t* overflow,
+                            void* stream);
+/* rsb_bn_stats_finalize on a two-plane z: the batch sums of hi + lo and of its square are accumulated in fp64 from the first add.
+ * Same sums scratch, outputs and running-stat update; "_chained" as rsb_bn_stats_finalize_chained (sums zero on entry, left zeroed).
+ * overflow (optional): the pack's counter; while it is non-zero the running statistics and num_batches are left untouched. */
+int rsb_bn_stats_finalize_split(const void* z, int64_t plane, double* sums, const float* gamma, const float* beta, float* running_mean,
+                                float* running_var, int64_t* num_batches, float* mean, float* invstd, float* scale, float* shift, int64_t M,
+                                int32_t C, float eps, float momentum, const int32_t* overflow, void* stream);
+int rsb_bn_stats_finalize_split_chained(const void* z, int64_t plane, double* sums, const float* gamma, const float* beta, float* running_mean,
+                                        float* running_var, int64_t* num_batches, float* mean, float* invstd, float* scale, float* shift,
+                                        int64_t M, int32_t C, float eps, float momentum, const int32_t* overflow, void* stream);
+/* y = relu?(z*scale + shift (+ residual)) in fp32 from two-plane z / residual, written as a (hi, lo) pair */
+int rsb_bn_apply_split(const void* z, int64_t z_plane, const float* scale, const float* shift, const void* residual, int64_t res_plane, void* y,
+                       int64_t y_plane, int64_t M, int32_t C, int32_t relu, void* stream);
+int rsb_bn_apply_split_chained(const void* z, int64_t z_plane, const float* scale, const float* shift, const void* residual, int64_t res_plane,
+                               void* y, int64_t y_plane, int64_t M, int32_t C, int32_t relu, void* stream);
+/* rsb_maxpool_backward for a two-plane x: every window's gradient goes to the FIRST position (row-major scan) whose hi + lo equals
+ * the window maximum, the element rsb_maxpool_nhwc_split forwarded (ATen's tie rule on the fp32 values). dy / dx single fp16;
+ * argmax_scratch (N*OH*OW*C bytes) is required. */
+int rsb_maxpool_backward_split(const void* x, int64_t x_plane, const void* dy, void* dx, void* argmax_scratch, int32_t N, int32_t H, int32_t W,
+                               int32_t C, int32_t k, int32_t s, int32_t p, void* stream);
+/* rsb_final_forward on two-plane dec5 activations: hi + lo contracted with the fp32 weights in fp32. overflow (optional): the pack's
+ * counter; while it is non-zero every logit is NaN, so that the step's loss and gradients are not finite (a guarded optimiser skips it) */
+int rsb_final_forward_split(const void* y5, int64_t plane, const float* w, const float* b, const int32_t* overflow, float* logits, int32_t N,
+                            int32_t HW, int32_t classes, void* stream);
+
 /* Weight gradient of the convolution described by `fwd` (same sources / segments / phases / tile space), on tensor cores:
  *   dw_packed[phase*Cout + co][k] = sum_pixels dy_phase[pixel][co] * x_segment(k)[pixel + (dh,dw)][k % 64-block]   (fp32)
  * i.e. the gradient in the forward kernel's packed weight layout (rsb_unpack_grads folds it back to OIHW).

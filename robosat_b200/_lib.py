@@ -175,7 +175,15 @@ SIGNATURES = {
     "rsb_pack_weights1": (ctypes.c_int, [_vp, _vp, _vp, _i64, _vp]),
     "rsb_unpack_grads": (ctypes.c_int, [_vp, _vp, _vp, _i64, _f32, _vp]),
     "rsb_unpack_grads_gather": (ctypes.c_int, [_vp, _vp, _vp, _vp, _i64, _f32, _vp]),
-    "rsb_wgrad_plan_create": (ctypes.c_int, [ctypes.POINTER(ConvDesc), _vp, _vp, ctypes.POINTER(_vp)]),
+    "rsb_pack_weights_split": (ctypes.c_int, [_vp, _vp, _vp, _i64, _i64, _f32, _vp, _vp]),
+    "rsb_pack_weights1_split": (ctypes.c_int, [_vp, _vp, _vp, _i64, _i64, _f32, _vp, _vp]),
+    "rsb_bn_stats_finalize_split": (ctypes.c_int, [_vp, _i64] + [_vp] * 10 + [_i64, _i32, _f32, _f32, _vp, _vp]),
+    "rsb_bn_stats_finalize_split_chained": (ctypes.c_int, [_vp, _i64] + [_vp] * 10 + [_i64, _i32, _f32, _f32, _vp, _vp]),
+    "rsb_bn_apply_split": (ctypes.c_int, [_vp, _i64, _vp, _vp, _vp, _i64, _vp, _i64, _i64, _i32, _i32, _vp]),
+    "rsb_bn_apply_split_chained": (ctypes.c_int, [_vp, _i64, _vp, _vp, _vp, _i64, _vp, _i64, _i64, _i32, _i32, _vp]),
+    "rsb_maxpool_backward_split": (ctypes.c_int, [_vp, _i64, _vp, _vp, _vp] + [_i32] * 7 + [_vp]),
+    "rsb_final_forward_split": (ctypes.c_int, [_vp, _i64, _vp, _vp, _vp, _vp, _i32, _i32, _i32, _vp]),
+    "rsb_wgrad_plan_create":(ctypes.c_int, [ctypes.POINTER(ConvDesc), _vp, _vp, ctypes.POINTER(_vp)]),
     "rsb_wgrad_plan_scratch_bytes": (_i64, [_vp]),
     "rsb_wgrad_plan_set_scratch": (ctypes.c_int, [_vp, _vp, _i64]),
     "rsb_wgrad_plan_destroy": (None, [_vp]),

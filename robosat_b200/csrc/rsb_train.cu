@@ -99,6 +99,7 @@ struct RedTail {
     float* dbeta;
     float eps, momentum, inv_scale;
     int self_clean;  // the last block leaves the accumulator slots and the arrival counter zeroed for the next call (no memset launch)
+    const int* frozen;  // strict plans: *frozen != 0 (weights past the plan's exponents) -> running statistics left untouched
 };
 
 __device__ __forceinline__ double red_slots(const double* sums, int which, int c, int C) {
@@ -868,6 +869,269 @@ __global__ void multi_axpy_kernel(const int64_t* __restrict__ table, float alpha
     for (int i = threadIdx.x; i < n; i += blockDim.x) dst[i] += alpha * src[i];
 }
 
+// ------------------------------------------------------------------------------------------------
+// Strict-precision training forward. Every forward activation is an fp16 (hi, lo) pair in two planes `plane` elements apart,
+// value = hi + lo (exact in fp32), with hi = half(v) and lo = half(v - hi) as the split convolutions write them.
+
+// v -> (hi, lo) of v * scale; `bad` when hi would not be a finite fp16 (|v * scale| rounds past 65504, or v is inf / NaN)
+__device__ __forceinline__ bool split_scaled(float v, float scale, __half& hi, __half& lo) {
+    const float vs = v * scale;
+    hi = __float2half_rn(vs);
+    lo = __float2half_rn(vs - __half2float(hi));
+    return !(fabsf(vs) < 65520.f);
+}
+
+__device__ __forceinline__ void split8(const float (&v)[8], __half* hi, __half* lo) {
+    __align__(16) __half h[8];
+    __align__(16) __half l[8];
+#pragma unroll
+    for (int e = 0; e < 8; ++e) {
+        h[e] = __float2half_rn(v[e]);
+        l[e] = __float2half_rn(v[e] - __half2float(h[e]));
+    }
+    *reinterpret_cast<uint4*>(hi) = *reinterpret_cast<const uint4*>(h);
+    *reinterpret_cast<uint4*>(lo) = *reinterpret_cast<const uint4*>(l);
+}
+
+// 8 channels of a pair as fp32 values hi + lo
+__device__ __forceinline__ void load8_pair(const __half* p, int64_t plane, float (&v)[8]) {
+    float l[8];
+    load8(p, v);
+    load8(p + plane, l);
+#pragma unroll
+    for (int e = 0; e < 8; ++e) v[e] += l[e];
+}
+
+// fp32 master weights -> split packed operand [2][n] (hi plane, lo plane at + plane) of w * scale, scale = 2^e fixed per layer.
+// Elements whose scaled hi is not a finite fp16 are counted in *overflow (the plan's exponent no longer fits the weights).
+__global__ void pack_gather_split_kernel(const float* __restrict__ src, const int32_t* __restrict__ map, __half* __restrict__ dst, int64_t plane,
+                                         int64_t n, float scale, int* __restrict__ overflow) {
+    for (int64_t i = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x; i < n; i += static_cast<int64_t>(gridDim.x) * blockDim.x) {
+        const int4 m = __ldg(reinterpret_cast<const int4*>(map) + i);
+        float v = 0.f;
+        if (m.x >= 0) v += src[m.x];
+        if (m.y >= 0) v += src[m.y];
+        if (m.z >= 0) v += src[m.z];
+        if (m.w >= 0) v += src[m.w];
+        __half h, l;
+        if (split_scaled(v, scale, h, l)) atomicAdd(overflow, 1);
+        dst[i] = h;
+        dst[plane + i] = l;
+    }
+}
+
+__global__ void pack_gather1_split_kernel(const float* __restrict__ src, const int32_t* __restrict__ map, __half* __restrict__ dst, int64_t plane,
+                                          int64_t n8, float scale, int* __restrict__ overflow) {
+    for (int64_t i = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x; i < n8; i += static_cast<int64_t>(gridDim.x) * blockDim.x) {
+        const int4 m0 = __ldg(reinterpret_cast<const int4*>(map) + 2 * i);
+        const int4 m1 = __ldg(reinterpret_cast<const int4*>(map) + 2 * i + 1);
+        const int idx[8] = {m0.x, m0.y, m0.z, m0.w, m1.x, m1.y, m1.z, m1.w};
+        __align__(16) __half h[8];
+        __align__(16) __half l[8];
+        int bad = 0;
+#pragma unroll
+        for (int j = 0; j < 8; ++j) bad += split_scaled(idx[j] >= 0 ? __ldg(src + idx[j]) : 0.f, scale, h[j], l[j]) ? 1 : 0;
+        if (bad) atomicAdd(overflow, bad);
+        *reinterpret_cast<uint4*>(dst + 8 * i) = *reinterpret_cast<const uint4*>(h);
+        *reinterpret_cast<uint4*>(dst + plane + 8 * i) = *reinterpret_cast<const uint4*>(l);
+    }
+}
+
+// BatchNorm finalize of one channel from the folded slot sums (what channel_reduce_kernel<0>'s last block does)
+__device__ __forceinline__ void bn_finalize_channel(double* sums, int c, int C, double dM, const RedTail& tail) {
+    const double t0 = red_slots(sums, 0, c, C), t1 = red_slots(sums, 1, c, C);
+    const double mean = t0 / dM;
+    double var = t1 / dM - mean * mean;
+    if (var < 0) var = 0;
+    const float invstd = static_cast<float>(1.0 / sqrt(var + static_cast<double>(tail.eps)));
+    const float sc = tail.gamma[c] * invstd;
+    tail.mean[c] = static_cast<float>(mean);
+    tail.invstd[c] = invstd;
+    tail.scale[c] = sc;
+    tail.shift[c] = tail.beta[c] - static_cast<float>(mean) * sc;
+    if (tail.running_mean && !(tail.frozen && *tail.frozen)) {
+        const double unbiased = dM > 1 ? var * dM / (dM - 1.0) : var;
+        tail.running_mean[c] = (1.f - tail.momentum) * tail.running_mean[c] + tail.momentum * static_cast<float>(mean);
+        tail.running_var[c] = (1.f - tail.momentum) * tail.running_var[c] + tail.momentum * static_cast<float>(unbiased);
+    }
+    if (tail.self_clean) {
+#pragma unroll
+        for (int sl = 0; sl < kRedSlots; ++sl) {
+            sums[(static_cast<int64_t>(sl) * 2 + 0) * C + c] = 0.0;
+            sums[(static_cast<int64_t>(sl) * 2 + 1) * C + c] = 0.0;
+        }
+    }
+}
+
+// Batch statistics of a two-plane z: per-channel sums of v = hi + lo and of v*v, accumulated in fp64 from the first add on
+// (fp32 partial sums would cost the statistics the precision the split forward buys), same slots / last-block finalize as
+// channel_reduce_kernel<0>. Thread mapping as there: C/8 threads per row, 256/(C/8) rows per iteration.
+__global__ void __launch_bounds__(256) bn_stats_split_kernel(const __half* __restrict__ z, int64_t plane, double* __restrict__ sums, int64_t M, int C,
+                                                             const RedTail tail) {
+    __shared__ double sh0[256 * 8];
+    __shared__ double sh1[256 * 8];
+    pdl_sync();
+    const int tpr = C / 8;
+    const int rows_per_iter = 256 / tpr;
+    const int col = (threadIdx.x % tpr) * 8;
+    const int rsub = threadIdx.x / tpr;
+    double acc0[8], acc1[8];
+#pragma unroll
+    for (int i = 0; i < 8; ++i) acc0[i] = acc1[i] = 0.0;
+    const int64_t step = static_cast<int64_t>(gridDim.x) * rows_per_iter;
+    auto fold = [&](const float (&v)[8]) {
+#pragma unroll
+        for (int i = 0; i < 8; ++i) {
+            const double d = static_cast<double>(v[i]);
+            acc0[i] += d;
+            acc1[i] = fma(d, d, acc1[i]);
+        }
+    };
+    int64_t r = static_cast<int64_t>(blockIdx.x) * rows_per_iter + rsub;
+    for (; r + step < M; r += 2 * step) {
+        float v0[8], v1[8];
+        load8_pair(z + r * C + col, plane, v0);
+        load8_pair(z + (r + step) * C + col, plane, v1);
+        fold(v0);
+        fold(v1);
+    }
+    if (r < M) {
+        float v0[8];
+        load8_pair(z + r * C + col, plane, v0);
+        fold(v0);
+    }
+#pragma unroll
+    for (int i = 0; i < 8; ++i) {
+        sh0[threadIdx.x * 8 + i] = acc0[i];
+        sh1[threadIdx.x * 8 + i] = acc1[i];
+    }
+    __syncthreads();
+    double* s0 = sums + static_cast<int64_t>(blockIdx.x % kRedSlots) * 2 * C;
+    double* s1 = s0 + C;
+    for (int c = threadIdx.x; c < C; c += blockDim.x) {
+        const int t0 = c / 8, e = c % 8;
+        double a0 = 0.0, a1 = 0.0;
+        for (int g = 0; g < rows_per_iter; ++g) {
+            a0 += sh0[(g * tpr + t0) * 8 + e];
+            a1 += sh1[(g * tpr + t0) * 8 + e];
+        }
+        atomicAdd(&s0[c], a0);
+        atomicAdd(&s1[c], a1);
+    }
+    __shared__ bool is_last;
+    __threadfence();
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        unsigned* counter = reinterpret_cast<unsigned*>(sums + static_cast<int64_t>(kRedSlots) * 2 * C);
+        is_last = atomicAdd(counter, 1u) == gridDim.x - 1;
+    }
+    __syncthreads();
+    if (!is_last) return;
+    __threadfence();
+    if (threadIdx.x == 0 && tail.num_batches && !(tail.frozen && *tail.frozen)) *tail.num_batches += 1;
+    for (int c = threadIdx.x; c < C; c += blockDim.x) bn_finalize_channel(sums, c, C, static_cast<double>(M), tail);
+    if (tail.self_clean && threadIdx.x == 0) *reinterpret_cast<unsigned*>(sums + static_cast<int64_t>(kRedSlots) * 2 * C) = 0u;
+}
+
+// y = relu?(z*scale + shift (+ res)) in fp32 from two-plane z and residual, written as a (hi, lo) pair. Channel mapping as
+// bn_apply_kernel (every thread keeps the same 8 channels for its whole loop).
+__global__ void bn_apply_split_kernel(const __half* __restrict__ z, int64_t zplane, const float* __restrict__ scale, const float* __restrict__ shift,
+                                      const __half* __restrict__ res, int64_t rplane, __half* __restrict__ y, int64_t yplane, int64_t M, int C,
+                                      int relu) {
+    pdl_sync();
+    const int C8 = C / 8;
+    const int64_t total = M * C8;
+    const int64_t i0 = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x;
+    const int col = static_cast<int>(i0 % C8) * 8;
+    float sc[8], sh[8];
+#pragma unroll
+    for (int e = 0; e < 8; ++e) {
+        sc[e] = scale[col + e];
+        sh[e] = shift[col + e];
+    }
+    const int64_t stride = static_cast<int64_t>(gridDim.x) * blockDim.x;
+    for (int64_t i = i0; i < total; i += stride) {
+        float v[8], r[8];
+        load8_pair(z + i * 8, zplane, v);
+        if (res) load8_pair(res + i * 8, rplane, r);
+#pragma unroll
+        for (int e = 0; e < 8; ++e) {
+            float o = fmaf(v[e], sc[e], sh[e]);
+            if (res) o += r[e];
+            v[e] = relu ? fmaxf(o, 0.f) : o;
+        }
+        split8(v, y + i * 8, y + yplane + i * 8);
+    }
+}
+
+// max-pool arg-max of two-plane x: the window position (dy*k + dx, row-major scan) of the FIRST element whose hi + lo equals the
+// window's maximum -- ties, including pairs whose hi planes tie and whose lo planes decide, resolve like ATen's max_pool2d
+// (first maximum in scan order) on the fp32 values. rsb_maxpool_nhwc_split takes its maximum over the same values.
+__global__ void maxpool_argmax_split_kernel(const __half* __restrict__ x, int64_t plane, uint8_t* __restrict__ idx, int N, int H, int W, int C, int k,
+                                            int s, int p, int OH, int OW) {
+    const int C8 = C / 8;
+    const int64_t total = static_cast<int64_t>(N) * OH * OW * C8;
+    for (int64_t i = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x; i < total; i += static_cast<int64_t>(gridDim.x) * blockDim.x) {
+        const int c8 = static_cast<int>(i % C8);
+        int64_t r = i / C8;
+        const int ow = static_cast<int>(r % OW);
+        r /= OW;
+        const int oh = static_cast<int>(r % OH);
+        const int n = static_cast<int>(r / OH);
+        float best[8];
+        uint32_t pos[8];
+        bool any = false;
+        for (int dyy = 0; dyy < k; ++dyy) {
+            const int hh = oh * s - p + dyy;
+            if (hh < 0 || hh >= H) continue;
+            for (int dxx = 0; dxx < k; ++dxx) {
+                const int ww = ow * s - p + dxx;
+                if (ww < 0 || ww >= W) continue;
+                float v[8];
+                load8_pair(x + ((static_cast<int64_t>(n) * H + hh) * W + ww) * C + c8 * 8, plane, v);
+                const uint32_t q = static_cast<uint32_t>(dyy * k + dxx);
+#pragma unroll
+                for (int e = 0; e < 8; ++e) {
+                    if (!any || v[e] > best[e]) {
+                        best[e] = v[e];
+                        pos[e] = q;
+                    }
+                }
+                any = true;
+            }
+        }
+        uint2 o;
+        o.x = pos[0] | (pos[1] << 8) | (pos[2] << 16) | (pos[3] << 24);
+        o.y = pos[4] | (pos[5] << 8) | (pos[6] << 16) | (pos[7] << 24);
+        *reinterpret_cast<uint2*>(idx + i * 8) = o;
+    }
+}
+
+// final 1x1 conv forward on two-plane dec5 activations: the fp32 values hi + lo contracted with the fp32 weights in fp32.
+// *overflow != 0: the plan's packed weights are not finite, and neither are the logits (NaN): the loss and the gradients of the
+// step follow, so the guarded optimiser skips it (a ReLU may have turned the non-finite activations into finite garbage on the way)
+__global__ void final_fwd_split_kernel(const __half* __restrict__ y5, int64_t plane, const float* __restrict__ w, const float* __restrict__ b,
+                                       const int* __restrict__ overflow, float* __restrict__ logits, int64_t P, int64_t HW, int classes) {
+    const bool poisoned = overflow && *overflow;
+    for (int64_t i = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x; i < P; i += static_cast<int64_t>(gridDim.x) * blockDim.x) {
+        float v[32];
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+            float t[8];
+            load8_pair(y5 + i * 32 + j * 8, plane, t);
+#pragma unroll
+            for (int e = 0; e < 8; ++e) v[j * 8 + e] = t[e];
+        }
+        const int64_t n = i / HW, pix = i % HW;
+        for (int k = 0; k < classes; ++k) {
+            float s = b[k];
+#pragma unroll
+            for (int c = 0; c < 32; ++c) s = fmaf(w[k * 32 + c], v[c], s);
+            logits[(n * classes + k) * HW + pix] = poisoned ? __int_as_float(0x7fc00000) : s;
+        }
+    }
+}
+
 }  // namespace rsb
 
 using namespace rsb;
@@ -1161,5 +1425,139 @@ extern "C" int rsb_multi_axpy(const int64_t* table, int32_t segments, float alph
     if (segments == 0) return RSB_OK;
     multi_axpy_kernel<<<static_cast<unsigned>(segments), 256, 0, static_cast<cudaStream_t>(stream)>>>(table, alpha);
     RSB_LAUNCH_CHECK("multi_axpy launch");
+    return RSB_OK;
+}
+
+// ------------------------------------------------------------------------------------------------ strict-precision training forward
+// every entry point validates its arguments first (RSB_E_INVALID on any host), then needs an sm_100 device (RSB_E_NODEVICE)
+static bool bad_plane(const void* p, int64_t plane) { return !p || plane <= 0 || (plane % 8) || (reinterpret_cast<uintptr_t>(p) & 15); }
+
+static int pack_split_impl(const float* src, const int32_t* map, void* dst, int64_t plane, int64_t n, float scale, int32_t* overflow, void* stream,
+                           bool single) {
+    if (!src || !map || !dst || !overflow || n <= 0 || plane < n || !(scale > 0.f) || !isfinite(scale))
+        return set_error(RSB_E_INVALID, "pack_weights_split: bad arguments (plane >= n, scale a positive finite number)");
+    if (single && ((n % 8) || (plane % 8) || (reinterpret_cast<uintptr_t>(dst) & 15) || (reinterpret_cast<uintptr_t>(map) & 15)))
+        return set_error(RSB_E_INVALID, "pack_weights1_split: n and plane multiples of 8, map and dst 16B aligned");
+    int rc = rsb_device_ok();
+    if (rc != RSB_OK) return rc;
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    if (single)
+        pack_gather1_split_kernel<<<tr_blocks(n / 8, 256), 256, 0, st>>>(src, map, static_cast<__half*>(dst), plane, n / 8, scale, overflow);
+    else
+        pack_gather_split_kernel<<<tr_blocks(n, 256), 256, 0, st>>>(src, map, static_cast<__half*>(dst), plane, n, scale, overflow);
+    RSB_LAUNCH_CHECK("pack_weights_split launch");
+    return RSB_OK;
+}
+
+extern "C" int rsb_pack_weights_split(const float* src, const int32_t* map4, void* dst, int64_t plane, int64_t n, float scale, int32_t* overflow,
+                                      void* stream) {
+    return pack_split_impl(src, map4, dst, plane, n, scale, overflow, stream, false);
+}
+
+extern "C" int rsb_pack_weights1_split(const float* src, const int32_t* map1, void* dst, int64_t plane, int64_t n, float scale, int32_t* overflow,
+                                       void* stream) {
+    return pack_split_impl(src, map1, dst, plane, n, scale, overflow, stream, true);
+}
+
+static int bn_stats_split_impl(const void* z, int64_t plane, double* sums, const float* gamma, const float* beta, float* running_mean, float* running_var,
+                               int64_t* num_batches, float* mean, float* invstd, float* scale, float* shift, int64_t M, int32_t C, float eps,
+                               float momentum, const int32_t* overflow, void* stream, bool chained) {
+    if (bad_plane(z, plane) || !sums || !gamma || !beta || !mean || !invstd || !scale || !shift || M <= 0 || bad_c(C) || C < 64)
+        return set_error(RSB_E_INVALID, "bn_stats_finalize_split: bad arguments (C in 64..2048, power of two; plane a multiple of 8)");
+    int rc = rsb_device_ok();
+    if (rc != RSB_OK) return rc;
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    if (!chained) {
+        cudaError_t e = cudaMemsetAsync(sums, 0, sizeof(double) * (2 * C * kRedSlots + 2), st);
+        if (e != cudaSuccess) return set_cuda_error(e, "bn_stats_finalize_split memset");
+    }
+    RedTail tail = {};
+    tail.gamma = gamma;
+    tail.beta = beta;
+    tail.running_mean = running_mean;
+    tail.running_var = running_var;
+    tail.num_batches = num_batches;
+    tail.mean = mean;
+    tail.invstd = invstd;
+    tail.scale = scale;
+    tail.shift = shift;
+    tail.eps = eps;
+    tail.momentum = momentum;
+    tail.self_clean = chained ? 1 : 0;
+    tail.frozen = overflow;
+    cudaError_t e = launch_chained(chained, bn_stats_split_kernel, reduce_blocks(M, C), 256, st, static_cast<const __half*>(z), plane, sums, M,
+                                   static_cast<int>(C), tail);
+    if (e != cudaSuccess) return set_cuda_error(e, "bn_stats_finalize_split launch");
+    return RSB_OK;
+}
+
+extern "C" int rsb_bn_stats_finalize_split(const void* z, int64_t plane, double* sums, const float* gamma, const float* beta, float* running_mean,
+                                           float* running_var, int64_t* num_batches, float* mean, float* invstd, float* scale, float* shift, int64_t M,
+                                           int32_t C, float eps, float momentum, const int32_t* overflow, void* stream) {
+    return bn_stats_split_impl(z, plane, sums, gamma, beta, running_mean, running_var, num_batches, mean, invstd, scale, shift, M, C, eps, momentum,
+                               overflow, stream, false);
+}
+
+extern "C" int rsb_bn_stats_finalize_split_chained(const void* z, int64_t plane, double* sums, const float* gamma, const float* beta,
+                                                   float* running_mean, float* running_var, int64_t* num_batches, float* mean, float* invstd,
+                                                   float* scale, float* shift, int64_t M, int32_t C, float eps, float momentum,
+                                                   const int32_t* overflow, void* stream) {
+    return bn_stats_split_impl(z, plane, sums, gamma, beta, running_mean, running_var, num_batches, mean, invstd, scale, shift, M, C, eps, momentum,
+                               overflow, stream, true);
+}
+
+static int bn_apply_split_impl(const void* z, int64_t z_plane, const float* scale, const float* shift, const void* residual, int64_t res_plane, void* y,
+                               int64_t y_plane, int64_t M, int32_t C, int32_t relu, void* stream, bool chained) {
+    if (bad_plane(z, z_plane) || bad_plane(y, y_plane) || (residual && bad_plane(residual, res_plane)) || !scale || !shift || M <= 0 || C <= 0 ||
+        (C % 8) || (256 % (C / 8 > 256 ? 256 : C / 8)))
+        return set_error(RSB_E_INVALID, "bn_apply_split: bad arguments (C a multiple of 8 with C/8 dividing 256; planes multiples of 8)");
+    int rc = rsb_device_ok();
+    if (rc != RSB_OK) return rc;
+    cudaError_t e = launch_chained(chained, bn_apply_split_kernel, tr_blocks(M * (C / 8), 256), 256, static_cast<cudaStream_t>(stream),
+                                   static_cast<const __half*>(z), z_plane, scale, shift, static_cast<const __half*>(residual), res_plane,
+                                   static_cast<__half*>(y), y_plane, M, static_cast<int>(C), static_cast<int>(relu));
+    if (e != cudaSuccess) return set_cuda_error(e, "bn_apply_split launch");
+    return RSB_OK;
+}
+
+extern "C" int rsb_bn_apply_split(const void* z, int64_t z_plane, const float* scale, const float* shift, const void* residual, int64_t res_plane,
+                                  void* y, int64_t y_plane, int64_t M, int32_t C, int32_t relu, void* stream) {
+    return bn_apply_split_impl(z, z_plane, scale, shift, residual, res_plane, y, y_plane, M, C, relu, stream, false);
+}
+
+extern "C" int rsb_bn_apply_split_chained(const void* z, int64_t z_plane, const float* scale, const float* shift, const void* residual,
+                                          int64_t res_plane, void* y, int64_t y_plane, int64_t M, int32_t C, int32_t relu, void* stream) {
+    return bn_apply_split_impl(z, z_plane, scale, shift, residual, res_plane, y, y_plane, M, C, relu, stream, true);
+}
+
+extern "C" int rsb_maxpool_backward_split(const void* x, int64_t x_plane, const void* dy, void* dx, void* argmax_scratch, int32_t N, int32_t H,
+                                          int32_t W, int32_t C, int32_t k, int32_t s, int32_t p, void* stream) {
+    if (bad_plane(x, x_plane) || !dy || !dx || !argmax_scratch || N <= 0 || H <= 0 || W <= 0 || C <= 0 || (C % 8) || k < 1 || k > 15 || s < 1 ||
+        p < 0 || 2 * p > k)
+        return set_error(RSB_E_INVALID, "maxpool_backward_split: bad arguments (argmax scratch required; C and x_plane multiples of 8)");
+    int rc = rsb_device_ok();
+    if (rc != RSB_OK) return rc;
+    const int OH = (H + 2 * p - k) / s + 1, OW = (W + 2 * p - k) / s + 1;
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    uint8_t* idx = static_cast<uint8_t*>(argmax_scratch);
+    maxpool_argmax_split_kernel<<<tr_blocks(static_cast<int64_t>(N) * OH * OW * (C / 8), 256), 256, 0, st>>>(static_cast<const __half*>(x), x_plane,
+                                                                                                            idx, N, H, W, C, k, s, p, OH, OW);
+    RSB_LAUNCH_CHECK("maxpool_argmax_split launch");
+    maxpool_bwd_gather_kernel<<<tr_blocks(static_cast<int64_t>(N) * H * W * (C / 8), 256), 256, 0, st>>>(
+        idx, static_cast<const __half*>(dy), static_cast<__half*>(dx), N, H, W, C, k, s, p, OH, OW);
+    RSB_LAUNCH_CHECK("maxpool_bwd_gather launch");
+    return RSB_OK;
+}
+
+extern "C" int rsb_final_forward_split(const void* y5, int64_t plane, const float* w, const float* b, const int32_t* overflow, float* logits,
+                                       int32_t N, int32_t HW, int32_t classes, void* stream) {
+    if (bad_plane(y5, plane) || !w || !b || !logits || N <= 0 || HW <= 0 || classes < 1 || classes > 8)
+        return set_error(RSB_E_INVALID, "final_forward_split: bad arguments");
+    int rc = rsb_device_ok();
+    if (rc != RSB_OK) return rc;
+    const int64_t P = static_cast<int64_t>(N) * HW;
+    final_fwd_split_kernel<<<tr_blocks(P, 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(static_cast<const __half*>(y5), plane, w, b, overflow, logits,
+                                                                                             P, HW, classes);
+    RSB_LAUNCH_CHECK("final_forward_split launch");
     return RSB_OK;
 }

@@ -14,9 +14,14 @@ Replaces what `outputs = net(images); loss.backward()` does in the reference's h
 The engine only builds buffers, descriptors and two op lists (`fwd_ops`, `bwd_ops`); an executor replays them. The GPU
 executor calls the C ABI; tests/emulate.py replays the same lists on the CPU to check the host logic against autograd.
 Activation gradients are fp16 and carry `loss_scale`; parameter gradients are fp32 and unscaled.
+
+precision="strict" (opt-in; RSB_TRAIN_PRECISION) keeps every forward activation as an fp16 (hi, lo) pair, like the strict inference
+plan: split convolutions, BatchNorm statistics of hi + lo in fp64, BN apply / max pool / final 1x1 on the fp32 values hi + lo. The
+backward is the fast one on the hi planes, with every ReLU mask and max-pool arg-max taken from what the strict forward applied.
 """
 
 import ctypes
+import math
 import os
 from collections import OrderedDict
 
@@ -24,13 +29,26 @@ import numpy as np
 import torch
 
 from robosat_b200 import _lib
-from robosat_b200._lib import ConvSrc
+from robosat_b200._lib import ConvDesc, ConvSrc
 
 # BatchNorm kernels chained by programmatic dependent launch, accumulators cleaned by the kernels themselves (no memset launches)
 TRAIN_GRAPH = os.environ.get("RSB_TRAIN_GRAPH", "1") == "1"  # forward / backward op lists replayed from CUDA graphs
 CONV_STATS = os.environ.get("RSB_CONV_STATS", "1") == "1"  # BatchNorm batch sums from the conv epilogue (profiles/r2_train.md)
 BN_CHAINED = os.environ.get("RSB_BN_CHAINED", "1") == "1"  # measured: 17.77 vs 18.03 ms per cfg-3 step (profiles/r2_train.md)
 from robosat_b200.engine import ConvOp, _src_dense, _src_parity, make_conv_desc
+
+TRAIN_PRECISIONS = ("fast", "strict")
+# strict plans scale every forward weight layout by a power of two fixed when the plan is built: its largest |w| lands in
+# [2^9, 2^10), so the weights may grow 64x before a scaled hi overflows fp16 (counted on the device; the owner rebuilds the plan)
+STRICT_WEIGHT_EXP = 9
+
+
+def default_train_precision():
+    """`fast` (single fp16 forward activations) unless RSB_TRAIN_PRECISION=strict (hi/lo fp16 pairs: fp32-class forward)"""
+    p = os.environ.get("RSB_TRAIN_PRECISION", "fast").lower()
+    if p not in TRAIN_PRECISIONS:
+        raise ValueError("RSB_TRAIN_PRECISION must be one of %s" % (TRAIN_PRECISIONS,))
+    return p
 
 RESNET50_BLOCKS = (3, 4, 6, 3)
 BN_EPS = 1e-5
@@ -156,11 +174,20 @@ class Unit:
 
 
 class UNetTrainEngine:
-    def __init__(self, params, num_classes, batch, height, width, device="cuda", loss_scale=4096.0, plan_only=False):
+    def __init__(self, params, num_classes, batch, height, width, device="cuda", loss_scale=4096.0, plan_only=False, precision=None):
         """params: name -> fp32 tensor on `device` with the reference's state_dict names WITHOUT the `module.` prefix
         (weights, BN affine + running stats + num_batches_tracked). They are read (and the BN buffers updated) in place.
-        Gradients are written to `self.grads[name]` (fp32, zeroed at the start of every backward)."""
+        Gradients are written to `self.grads[name]` (fp32, zeroed at the start of every backward).
+
+        precision: "fast" (single fp16 forward activations and weights), "strict" (every forward activation an fp16 (hi, lo) pair,
+        split convolutions with three MMAs per K step, BatchNorm statistics in fp64 from hi + lo: train-mode logits, batch
+        statistics, ReLU masks and max-pool arg-maxes at fp32 level; the backward is the fast one, reading the hi planes) or None
+        (RSB_TRAIN_PRECISION, default fast)."""
         assert height % 64 == 0 and width % 64 == 0
+        self.precision = default_train_precision() if precision is None else precision
+        if self.precision not in TRAIN_PRECISIONS:
+            raise ValueError("precision must be one of %s, not %r" % (TRAIN_PRECISIONS, precision))
+        self.strict = self.precision == "strict"
         self.plan_only = plan_only
         if not plan_only:
             _lib.require_device()
@@ -184,6 +211,12 @@ class UNetTrainEngine:
         self.units = OrderedDict()
         self.feats = OrderedDict()
         self.relu_outs = OrderedDict()  # name -> (post-ReLU activation buffer, logical NHWC shape): masks for tests / debugging
+        # strict: forward weight layouts packed as (hi, lo) planes of w * 2^e, one exponent per layout; weights past it are counted
+        self.split_pack_list = []  # (wname, map, packed fp16 [2][n], 2^e, one source per element?)
+        self.exponents = OrderedDict()  # unit name -> e (the unit's forward descriptor has acc_scale = 2^-e)
+        self._pair_planes = {}  # data_ptr -> plane stride of every two-plane forward activation buffer
+        self.overflow = self._buf(1, dtype=torch.int32) if self.strict else None
+        self._overflow_host, self._overflow_event = None, None
         self._build()
 
     # ---------------------------------------------------------------- allocation helpers
@@ -215,6 +248,50 @@ class UNetTrainEngine:
                 off += n
         return self.grads[name]
 
+    def _act(self, *shape):
+        """forward activation buffer: NHWC fp16, with a leading (hi, lo) plane axis in strict precision"""
+        if not self.strict:
+            return self._buf(*shape)
+        t = self._buf(2, *shape)
+        self._pair_planes[t.data_ptr()] = t.numel() // 2
+        return t
+
+    def _plane(self, t):
+        return self._pair_planes.get(t.data_ptr(), 0) if t is not None else 0
+
+    def _hi(self, t):
+        """the single fp16 view the backward kernels read: the hi plane of a two-plane activation (the buffer itself otherwise)"""
+        return t[0] if self._plane(t) else t
+
+    def _dense(self, t, N, H, W, C):
+        return _src_dense(t, N, H, W, C, self._plane(t))
+
+    def _parity(self, t, N, H, W, C, ph, pw):
+        return _src_parity(t, N, H, W, C, ph, pw, self._plane(t))
+
+    def _scratch(self):
+        """one fp32 scratch tile per SM for the K-chunked split convolutions, shared by all layers (launches are stream ordered)"""
+        if getattr(self, "_scratch_buf", None) is None:
+            n = 148 * 128 * 256 if self.plan_only else int(_lib.load().rsb_conv_scratch_bytes(256)) // 4
+            self._scratch_buf = self._buf(n, dtype=torch.float32)
+        return self._scratch_buf
+
+    def _packed_split(self, name, wname, m):
+        """strict forward layout of `wname` (m: device map [n, 4]): fp16 [2][n] (hi, lo) of the packed weights times 2^e, refreshed
+        by pack_all every step. e is fixed here from the current weights (it is baked into the conv's acc_scale and the captured
+        graphs)."""
+        src = self.params[wname].detach().reshape(-1)
+        mm = m.long()
+        vals = torch.where(mm >= 0, src[mm.clamp_min(0)], torch.zeros((), device=src.device)).sum(1)
+        amax = float(vals.abs().max())
+        e = STRICT_WEIGHT_EXP - int(math.floor(math.log2(amax))) if math.isfinite(amax) and amax > 0 else 0
+        single = bool((m[:, 1:] < 0).all())
+        dm = self._dev(m[:, 0], torch.int32) if single else m
+        dst = self._buf(2, m.shape[0])
+        self.split_pack_list.append((wname, dm, dst, 2.0 ** e, single))
+        self.exponents[name] = e
+        return dst, 2.0 ** -e
+
     def _conv_op(self, name, desc):
         return ConvOp(name, desc, (), create_plan=not self.plan_only)
 
@@ -244,11 +321,27 @@ class UNetTrainEngine:
         u.wname = wname
         w = self.params[wname]
         u.wshape = tuple(w.shape)
-        u.w_packed, u.fwd_map = self._packed(wname, fwd_map)
         K = 64 * sum(s[3] for s in segs)
-        wp = u.w_packed.view(phases * cout, K)
-        u.desc = make_conv_desc(srcs, segs, wp, None, cout, phases, tile_space, out, out_pitches, out_scale=out_scale, relu=relu,
-                                out_offset_elems=out_offset, residual=residual)
+        if self.strict:
+            # split forward (raw z, or ReLU in the epilogue); the weight gradient runs on a single-plane copy of the descriptor
+            # (hi planes of the sources, which are the buffer bases)
+            u.fwd_map = self._dev(fwd_map, torch.int32)
+            u.w_packed, acc_scale = self._packed_split(name, wname, u.fwd_map)
+            u.desc = make_conv_desc(srcs, segs, u.w_packed.view(2, phases * cout, K), None, cout, phases, tile_space, out, out_pitches,
+                                    out_scale=out_scale, relu=relu, out_offset_elems=out_offset, residual=residual, split=True,
+                                    acc_scale=acc_scale, out_plane=self._plane(out), res_plane=self._plane(residual), scratch=self._scratch())
+            u.wdesc = ConvDesc.from_buffer_copy(u.desc)
+            wd = u.wdesc
+            wd.split, wd.acc_scale, wd.out_plane, wd.res_plane, wd.kchunk, wd.scratch, wd.scratch_bytes = 0, 1.0, 0, 0, 0, None, 0
+            for i in range(wd.nsrc):
+                wd.srcs[i].plane = 0
+            stats = False  # conv-epilogue statistics are single-plane only: the strict plan reduces hi + lo in rsb_bn_stats_finalize_split
+        else:
+            u.w_packed, u.fwd_map = self._packed(wname, fwd_map)
+            wp = u.w_packed.view(phases * cout, K)
+            u.desc = make_conv_desc(srcs, segs, wp, None, cout, phases, tile_space, out, out_pitches, out_scale=out_scale, relu=relu,
+                                    out_offset_elems=out_offset, residual=residual)
+            u.wdesc = u.desc
         u.stats, u.stats_rows = None, 0
         if stats and CONV_STATS:
             d = u.desc
@@ -310,13 +403,22 @@ class UNetTrainEngine:
 
     def _bn(self, prefix, z, M, C, conv=None):
         b = Unit(prefix)
-        b.prefix, b.z, b.M, b.C = prefix, z, M, C
+        # b.z: what the backward reads (the hi plane in strict precision); b.zpair / b.zplane: the two-plane forward value
+        b.prefix, b.z, b.M, b.C = prefix, self._hi(z), M, C
+        b.zpair, b.zplane = z, self._plane(z)
         b.partials, b.partial_rows = (conv.stats, conv.stats_rows) if conv is not None and conv.stats is not None else (None, 0)
         b.sums = self._buf(20 * C, dtype=torch.float64)  # 8 accumulator slots x {sum0, sum1} x C, arrival counter, backward coefficients
         b.mean, b.invstd, b.scale, b.shift = (self._buf(C, dtype=torch.float32) for _ in range(4))
         return b
 
     def _bn_fwd_ops(self, b, y, residual, relu):
+        if self.strict:
+            # statistics of hi + lo (fp64), apply in fp32 to a (hi, lo) pair. The backward masks by y (hi plane), never by a mask
+            # re-derived from single-plane z
+            self.fwd_ops.append(("bn_stats_split", b))
+            self.fwd_ops.append(("bn_apply_split", b, residual, y, relu))
+            b.plain_relu_y = None
+            return
         self.fwd_ops.append(("bn_stats", b))
         self.fwd_ops.append(("bn_finalize", b))
         self.fwd_ops.append(("bn_apply", b, residual, y, relu))
@@ -334,26 +436,27 @@ class UNetTrainEngine:
 
         # ---- stem
         self.x_in = None
-        self.s2d = self._buf(N, H2, W2 + 4, 16)
+        self.s2d = self._act(N, H2, W2 + 4, 16)
         self.fwd_ops.append(("pack_all",))
-        self.fwd_ops.append(("prepass",))
+        self.fwd_ops.append(("prepass_split",) if self.strict else ("prepass",))
         Wp = W2 + 4
-        z0 = self._buf(N, H2, W2, 64)
-        y0 = self._buf(N, H2, W2, 64)
-        src = ConvSrc(self.s2d.data_ptr(), 16, Wp * 16, H2 * Wp * 16, 64, W2, H2, N)
+        z0 = self._act(N, H2, W2, 64)
+        y0 = self._act(N, H2, W2, 64)
+        src = ConvSrc(self.s2d.data_ptr(), 16, Wp * 16, H2 * Wp * 16, 64, W2, H2, N, self._plane(self.s2d))
         stem = self._add_unit("stem", "resnet.conv1.weight", map_stem_fwd(tuple(P["resnet.conv1.weight"].shape)), [src],
                               [(0, t - 2, 0, 1) for t in range(4)], 64, 1, (W2, H2, N), z0, dense(H2, W2, 64), stats=True)
         bn0 = self._bn("resnet.bn1", z0, N * H2 * W2, 64, conv=stem)
         self._bn_fwd_ops(bn0, y0, None, True)
-        p0 = self._buf(N, H4, W4, 64)
-        self.fwd_ops.append(("maxpool", y0, p0, N, H2, W2, 64, 3, 2, 1))
+        p0 = self._act(N, H4, W4, 64)
+        self.fwd_ops.append(("maxpool_split" if self.strict else "maxpool", y0, p0, N, H2, W2, 64, 3, 2, 1))
         self.feats["stem"] = (y0, (N, H2, W2, 64))
         self.relu_outs["stem"] = (y0, (N, H2, W2, 64))
         self.feats["enc0"] = (p0, (N, H4, W4, 64))
         d_p0 = self._buf(N, H4, W4, 64)   # gradient w.r.t. p0, produced by layer1.0's backward
         d_y0 = self._buf(N, H2, W2, 64)
         dz0 = self._buf(N, H2, W2, 64)
-        bwd.append([("maxpool_bwd", y0, d_p0, d_y0, N, H2, W2, 64, 3, 2, 1), ("bn_bwd", bn0, d_y0, y0, dz0, None)] + self._wgrad_ops(stem, dz0))
+        bwd.append([("maxpool_bwd_split" if self.strict else "maxpool_bwd", y0, d_p0, d_y0, N, H2, W2, 64, 3, 2, 1),
+                    ("bn_bwd", bn0, d_y0, self._hi(y0), dz0, None)] + self._wgrad_ops(stem, dz0))
 
         # ---- encoder
         cur, curC, curH, curW, d_cur = p0, 64, H4, W4, d_p0
@@ -368,31 +471,31 @@ class UNetTrainEngine:
                 has_ds = (p + ".downsample.0.weight") in P
                 M_in, M_out = N * curH * curW, N * oH * oW
                 # forward
-                z1, y1 = self._buf(N, curH, curW, planes), self._buf(N, curH, curW, planes)
+                z1, y1 = self._act(N, curH, curW, planes), self._act(N, curH, curW, planes)
                 u1 = self._add_unit(p + ".conv1", p + ".conv1.weight", map_conv_fwd(tuple(P[p + ".conv1.weight"].shape)),
-                                    [_src_dense(cur, N, curH, curW, curC)], [(0, 0, 0, curC // 64)], planes, 1, (curW, curH, N), z1,
+                                    [self._dense(cur, N, curH, curW, curC)], [(0, 0, 0, curC // 64)], planes, 1, (curW, curH, N), z1,
                                     dense(curH, curW, planes), stats=True)
                 b1 = self._bn(p + ".bn1", z1, M_in, planes, conv=u1)
                 self._bn_fwd_ops(b1, y1, None, True)
-                z2, y2 = self._buf(N, oH, oW, planes), self._buf(N, oH, oW, planes)
+                z2, y2 = self._act(N, oH, oW, planes), self._act(N, oH, oW, planes)
                 if stride == 1:
-                    srcs2 = [_src_dense(y1, N, curH, curW, planes)]
+                    srcs2 = [self._dense(y1, N, curH, curW, planes)]
                     segs2 = [(0, kh - 1, kw - 1, planes // 64) for kh in range(3) for kw in range(3)]
                 else:
-                    srcs2 = [_src_parity(y1, N, curH, curW, planes, ph, pw) for ph in range(2) for pw in range(2)]
+                    srcs2 = [self._parity(y1, N, curH, curW, planes, ph, pw) for ph in range(2) for pw in range(2)]
                     segs2 = [(((kh - 1) % 2) * 2 + (kw - 1) % 2, (kh - 1) // 2, (kw - 1) // 2, planes // 64) for kh in range(3) for kw in range(3)]
                 u2 = self._add_unit(p + ".conv2", p + ".conv2.weight", map_conv_fwd(tuple(P[p + ".conv2.weight"].shape)), srcs2, segs2,
                                     planes, 1, (oW, oH, N), z2, dense(oH, oW, planes), stats=True)
                 b2 = self._bn(p + ".bn2", z2, M_out, planes, conv=u2)
                 self._bn_fwd_ops(b2, y2, None, True)
-                z3 = self._buf(N, oH, oW, outC)
+                z3 = self._act(N, oH, oW, outC)
                 u3 = self._add_unit(p + ".conv3", p + ".conv3.weight", map_conv_fwd(tuple(P[p + ".conv3.weight"].shape)),
-                                    [_src_dense(y2, N, oH, oW, planes)], [(0, 0, 0, planes // 64)], outC, 1, (oW, oH, N), z3, dense(oH, oW, outC),
+                                    [self._dense(y2, N, oH, oW, planes)], [(0, 0, 0, planes // 64)], outC, 1, (oW, oH, N), z3, dense(oH, oW, outC),
                                     stats=True)
                 b3 = self._bn(p + ".bn3", z3, M_out, outC, conv=u3)
                 if has_ds:
-                    zd, idt = self._buf(N, oH, oW, outC), self._buf(N, oH, oW, outC)
-                    sd_ = _src_dense(cur, N, curH, curW, curC) if stride == 1 else _src_parity(cur, N, curH, curW, curC, 0, 0)
+                    zd, idt = self._act(N, oH, oW, outC), self._act(N, oH, oW, outC)
+                    sd_ = self._dense(cur, N, curH, curW, curC) if stride == 1 else self._parity(cur, N, curH, curW, curC, 0, 0)
                     ud = self._add_unit(p + ".downsample", p + ".downsample.0.weight", map_conv_fwd(tuple(P[p + ".downsample.0.weight"].shape)),
                                         [sd_], [(0, 0, 0, curC // 64)], outC, 1, (oW, oH, N), zd, dense(oH, oW, outC),
                                         stats=True, stats_slot=1)
@@ -400,7 +503,7 @@ class UNetTrainEngine:
                     self._bn_fwd_ops(bd, idt, None, False)
                 else:
                     idt = cur
-                out = self._buf(N, oH, oW, outC)
+                out = self._act(N, oH, oW, outC)
                 self._bn_fwd_ops(b3, out, idt, True)
                 self.feats[p] = (out, (N, oH, oW, outC))
                 self.relu_outs[p + ".relu1"] = (y1, (N, curH, curW, planes))
@@ -411,13 +514,13 @@ class UNetTrainEngine:
                 # backward of this block (executed after all later blocks)
                 ops = []
                 dz3, g = self._buf(N, oH, oW, outC), self._buf(N, oH, oW, outC)
-                ops.append(("bn_bwd", b3, d_out, out, dz3, g))
+                ops.append(("bn_bwd", b3, d_out, self._hi(out), dz3, g))
                 ops += self._wgrad_ops(u3, dz3)
                 dy2 = self._buf(N, oH, oW, planes)
                 ops += self._dgrad(p + ".conv3.dgrad", p + ".conv3.weight", map_conv_dgrad(u3.wshape), [_src_dense(dz3, N, oH, oW, outC)],
                                    [(0, 0, 0, outC // 64)], planes, 1, (oW, oH, N), dy2, dense(oH, oW, planes))
                 dz2 = self._buf(N, oH, oW, planes)
-                ops.append(("bn_bwd", b2, dy2, y2, dz2, None))
+                ops.append(("bn_bwd", b2, dy2, self._hi(y2), dz2, None))
                 ops += self._wgrad_ops(u2, dz2)
                 dy1 = self._buf(N, curH, curW, planes)
                 if stride == 1:
@@ -429,7 +532,7 @@ class UNetTrainEngine:
                                        [(0, th - 1, tw - 1, planes // 64) for th in range(2) for tw in range(2)], planes, 4, (oW, oH, N), dy1,
                                        dense(curH, curW, planes), out_scale=(2, 2))
                 dz1 = self._buf(N, curH, curW, planes)
-                ops.append(("bn_bwd", b1, dy1, y1, dz1, None))
+                ops.append(("bn_bwd", b1, dy1, self._hi(y1), dz1, None))
                 ops += self._wgrad_ops(u1, dz1)
                 if has_ds:
                     dzd = self._buf(N, oH, oW, outC)
@@ -456,8 +559,8 @@ class UNetTrainEngine:
 
         # ---- center + decoder
         hp, wpx = h4 // 2, w4 // 2
-        pool4 = self._buf(N, hp, wpx, c4)
-        self.fwd_ops.append(("maxpool", enc4, pool4, N, h4, w4, c4, 2, 2, 0))
+        pool4 = self._act(N, hp, wpx, c4)
+        self.fwd_ops.append(("maxpool_split" if self.strict else "maxpool", enc4, pool4, N, h4, w4, c4, 2, 2, 0))
         d_pool4 = self._buf(N, hp, wpx, c4)
 
         dec_bwd = []
@@ -466,12 +569,12 @@ class UNetTrainEngine:
             """sources: [(tensor, C)]; d_sources: [(grad tensor, accumulate?)] receiving the input gradients"""
             wname = name + ".block.block.weight"
             wshape = tuple(P[wname].shape)
-            srcs = [_src_dense(t, N, lh, lw, c) for t, c in sources]
+            srcs = [self._dense(t, N, lh, lw, c) for t, c in sources]
             segs = [(si, th - 1, tw - 1, c // 64) for th in range(2) for tw in range(2) for si, (_, c) in enumerate(sources)]
             u = self._add_unit(name, wname, map_up_fwd(wshape), srcs, segs, cout, 4, (lw, lh, N), out, out_pitches, out_scale=(2, 2), relu=True,
                                out_offset=out_offset)
             # backward: g = d_out * (out > 0) in place over the whole buffer, wgrad, then one dgrad launch per source
-            ops = [("relu_bwd", d_out, None, out, d_out)]
+            ops = [("relu_bwd", d_out, None, self._hi(out), d_out)]
             ops += self._wgrad_ops(u, d_out)
             pad_co = -(-cout // 64) * 64
             oH, oW = 2 * lh, 2 * lw
@@ -486,24 +589,24 @@ class UNetTrainEngine:
             dec_bwd.append(ops)
             return u
 
-        center = self._buf(N, h4, w4, 256)
+        center = self._act(N, h4, w4, 256)
         d_center = self._buf(N, h4, w4, 256)
         decoder("center", [(pool4, c4)], hp, wpx, 256, center, dense(h4, w4, 256), d_center, dense(h4, w4, 256), [(d_pool4, False)])
-        dec0 = self._buf(N, h3, w3, 256)
+        dec0 = self._act(N, h3, w3, 256)
         d_dec0 = self._buf(N, h3, w3, 256)
         # d_enc4 receives the dec0 skip gradient first (plain write), then the max-pool gradient from center is added
         decoder("dec0", [(enc4, c4), (center, 256)], h4, w4, 256, dec0, dense(h3, w3, 256), d_dec0, dense(h3, w3, 256), [(d_enc4, False), (d_center, False)])
-        dec1 = self._buf(N, h2, w2, 256)
+        dec1 = self._act(N, h2, w2, 256)
         d_dec1 = self._buf(N, h2, w2, 256)
         decoder("dec1", [(enc3, c3), (dec0, 256)], h3, w3, 256, dec1, dense(h2, w2, 256), d_dec1, dense(h2, w2, 256), [(d_enc3, False), (d_dec0, False)])
-        dec2 = self._buf(N, h1, w1, 64)
+        dec2 = self._act(N, h1, w1, 64)
         d_dec2 = self._buf(N, h1, w1, 64)
         decoder("dec2", [(enc2, c2), (dec1, 256)], h2, w2, 64, dec2, dense(h1, w1, 64), d_dec2, dense(h1, w1, 64), [(d_enc2, False), (d_dec1, False)])
-        dec3 = self._buf(N, H2, W2, 128)
+        dec3 = self._act(N, H2, W2, 128)
         d_dec3 = self._buf(N, H2, W2, 128)
         decoder("dec3", [(enc1, c1), (dec2, 64)], h1, w1, 128, dec3, dense(H2, W2, 128), d_dec3, dense(H2, W2, 128), [(d_enc1, False), (d_dec2, False)])
         Wq = W + 4
-        dec4 = self._buf(N, H, Wq, 32)
+        dec4 = self._act(N, H, Wq, 32)
         d_dec4 = self._buf(N, H, Wq, 32)
         padded = (32, Wq * 32, H * Wq * 32)
         decoder("dec4", [(dec3, 128)], H2, W2, 32, dec4, padded, d_dec4, padded, [(d_dec3, False)], out_offset=32)
@@ -513,18 +616,18 @@ class UNetTrainEngine:
             self.relu_outs[nm] = (t, shp)
 
         # dec5: plain 3x3 on the W-padded dec4 buffer (window view), relu in the epilogue
-        y5 = self._buf(N, H, W, 32)
+        y5 = self._act(N, H, W, 32)
         d_y5 = self._buf(N, H, W, 32)
-        src5 = ConvSrc(dec4.data_ptr(), 32, Wq * 32, H * Wq * 32, 128, W, H, N)
+        src5 = ConvSrc(dec4.data_ptr(), 32, Wq * 32, H * Wq * 32, 128, W, H, N, self._plane(dec4))
         u5 = self._add_unit("dec5", "dec5.block.weight", map_window3_fwd(tuple(P["dec5.block.weight"].shape)), [src5],
                             [(0, kh - 1, 0, 2) for kh in range(3)], 32, 1, (W, H, N), y5, dense(H, W, 32), relu=True)
         self.feats["dec5"] = (y5, (N, H, W, 32))
         self.relu_outs["dec5"] = (y5, (N, H, W, 32))
         self.logits = self._buf(N, self.C, H, W, dtype=torch.float32)
-        self.fwd_ops.append(("final_fwd", y5, self.logits))
+        self.fwd_ops.append(("final_fwd_split" if self.strict else "final_fwd", y5, self.logits))
         self.final_acc = self._buf(self.C * 32 + 8, dtype=torch.float64)
 
-        ops5 = [("final_bwd", y5, d_y5), ("relu_bwd", d_y5, None, y5, d_y5)]
+        ops5 = [("final_bwd", self._hi(y5), d_y5), ("relu_bwd", d_y5, None, self._hi(y5), d_y5)]
         ops5 += self._wgrad_ops(u5, d_y5)
         ops5 += self._dgrad("dec5.dgrad", "dec5.block.weight", map_conv_dgrad(u5.wshape, pad_co_to=64), [_src_dense(d_y5, N, H, W, 32)],
                             [(0, kh - 1, kw - 1, 1) for kh in range(3) for kw in range(3)], 32, 1, (W, H, N), d_dec4, padded, out_offset=32)
@@ -535,7 +638,7 @@ class UNetTrainEngine:
             self.bwd_ops += ops
         # enc4's gradient = dec0 skip gradient (already in d_enc4) + max-pool backward of the center branch
         d_enc4_pool = self._buf(N, h4, w4, c4)
-        self.bwd_ops.append(("maxpool_bwd", enc4, d_pool4, d_enc4_pool, N, h4, w4, c4, 2, 2, 0))
+        self.bwd_ops.append(("maxpool_bwd_split" if self.strict else "maxpool_bwd", enc4, d_pool4, d_enc4_pool, N, h4, w4, c4, 2, 2, 0))
         self.bwd_ops.append(("relu_bwd", d_enc4, d_enc4_pool, None, d_enc4))  # plain sum (no mask)
         for ops in reversed(bwd):
             self.bwd_ops += ops
@@ -554,6 +657,10 @@ class UNetTrainEngine:
                 op[1].run(st)
             elif k == "pack_all":
                 self._run_pack_all(lib, st)
+                for w, m, d, scale, single in self.split_pack_list:
+                    n = d.shape[1]
+                    _lib.check((lib.rsb_pack_weights1_split if single else lib.rsb_pack_weights_split)(
+                        P[w].data_ptr(), m.data_ptr(), d.data_ptr(), n, n, scale, self.overflow.data_ptr(), st), "rsb_pack_weights_split[%s]" % w)
             elif k == "unpack_all":
                 # packed weight gradients (fp32 arena chunks) -> the flat OIHW gradient buffer: one launch per chunk
                 if self._unpack_all is None:
@@ -609,6 +716,19 @@ class UNetTrainEngine:
                                                      b.scale.data_ptr(), b.shift.data_ptr(), b.M, b.C, BN_EPS, BN_MOMENTUM, st), "rsb_bn_stats_finalize_chained")
             elif k == "bn_finalize":
                 pass  # fused into the bn_stats launch (kept as an op for the CPU emulation of the plan)
+            elif k == "bn_stats_split":
+                b = op[1]
+                pf = b.prefix
+                _lib.check((lib.rsb_bn_stats_finalize_split_chained if BN_CHAINED else lib.rsb_bn_stats_finalize_split)(
+                    b.zpair.data_ptr(), b.zplane, b.sums.data_ptr(), P[pf + ".weight"].data_ptr(), P[pf + ".bias"].data_ptr(),
+                    P[pf + ".running_mean"].data_ptr(), P[pf + ".running_var"].data_ptr(), P[pf + ".num_batches_tracked"].data_ptr(),
+                    b.mean.data_ptr(), b.invstd.data_ptr(), b.scale.data_ptr(), b.shift.data_ptr(), b.M, b.C, BN_EPS, BN_MOMENTUM,
+                    self.overflow.data_ptr(), st), "rsb_bn_stats_finalize_split")
+            elif k == "bn_apply_split":
+                _, b, res, y, relu = op
+                _lib.check((lib.rsb_bn_apply_split_chained if BN_CHAINED else lib.rsb_bn_apply_split)(
+                    b.zpair.data_ptr(), b.zplane, b.scale.data_ptr(), b.shift.data_ptr(), res.data_ptr() if res is not None else None,
+                    self._plane(res), y.data_ptr(), self._plane(y), b.M, b.C, 1 if relu else 0, st), "rsb_bn_apply_split")
             elif k == "bn_apply":
                 _, b, res, y, relu = op
                 _lib.check((lib.rsb_bn_apply_chained if BN_CHAINED else lib.rsb_bn_apply)(b.z.data_ptr(), b.scale.data_ptr(), b.shift.data_ptr(), res.data_ptr() if res is not None else None,
@@ -631,24 +751,41 @@ class UNetTrainEngine:
             elif k == "maxpool":
                 _, src, dst, n, h, w, c, kk, s, p = op
                 _lib.check(lib.rsb_maxpool_nhwc(src.data_ptr(), dst.data_ptr(), n, h, w, c, kk, s, p, st), "rsb_maxpool_nhwc")
-            elif k == "maxpool_bwd":
+            elif k in ("maxpool_bwd", "maxpool_bwd_split"):
                 _, xx, dy, dx, n, h, w, c, kk, s, p = op
                 scratch = self._pool_scratch.get(id(dx))
                 if scratch is None:
                     scratch = self._pool_scratch[id(dx)] = torch.empty(dy.numel(), dtype=torch.uint8, device=dx.device)
+                if k == "maxpool_bwd_split":
+                    _lib.check(lib.rsb_maxpool_backward_split(xx.data_ptr(), self._plane(xx), dy.data_ptr(), dx.data_ptr(), scratch.data_ptr(),
+                                                              n, h, w, c, kk, s, p, st), "rsb_maxpool_backward_split")
+                    continue
                 _lib.check(lib.rsb_maxpool_backward(xx.data_ptr(), dy.data_ptr(), dx.data_ptr(), scratch.data_ptr(), n, h, w, c, kk, s, p, st),
                            "rsb_maxpool_backward")
+            elif k == "maxpool_split":
+                _, src, dst, n, h, w, c, kk, s, p = op
+                _lib.check(lib.rsb_maxpool_nhwc_split(src.data_ptr(), self._plane(src), dst.data_ptr(), self._plane(dst), n, h, w, c, kk, s, p, st),
+                           "rsb_maxpool_nhwc_split")
             elif k == "wgrad":
                 _, u, dy = op
                 if not hasattr(u, "wgrad_plan"):
                     u.wgrad_plan = ctypes.c_void_p()
-                    _lib.check(lib.rsb_wgrad_plan_create(ctypes.byref(u.desc), dy.data_ptr() + 2 * u.out_offset, u.dw_packed.data_ptr(),
+                    _lib.check(lib.rsb_wgrad_plan_create(ctypes.byref(u.wdesc), dy.data_ptr() + 2 * u.out_offset, u.dw_packed.data_ptr(),
                                                          ctypes.byref(u.wgrad_plan)), "rsb_wgrad_plan_create[%s]" % u.name)
                     self._wgrad_scratch_for(u.wgrad_plan)
                 _lib.check(lib.rsb_wgrad_run(u.wgrad_plan, st), "rsb_wgrad_run[%s]" % u.name)
             elif k == "prepass":
                 kind = 0 if x.dtype == torch.float32 else 1
                 _lib.check(lib.rsb_prepass_s2d(x.data_ptr(), kind, self.s2d.data_ptr(), self.N, self.H, self.W, self._mean, self._std, st), "rsb_prepass_s2d")
+            elif k == "prepass_split":
+                kind = 0 if x.dtype == torch.float32 else 1
+                _lib.check(lib.rsb_prepass_s2d_split(x.data_ptr(), kind, self.s2d.data_ptr(), self._plane(self.s2d), self.N, self.H, self.W,
+                                                     self._mean, self._std, st), "rsb_prepass_s2d_split")
+            elif k == "final_fwd_split":
+                _, y5, logits = op
+                _lib.check(lib.rsb_final_forward_split(y5.data_ptr(), self._plane(y5), P["final.weight"].data_ptr(), P["final.bias"].data_ptr(),
+                                                       self.overflow.data_ptr(), logits.data_ptr(), self.N, self.H * self.W, self.C, st),
+                           "rsb_final_forward_split")
             elif k == "final_fwd":
                 _, y5, logits = op
                 _lib.check(lib.rsb_final_forward(y5.data_ptr(), P["final.weight"].data_ptr(), P["final.bias"].data_ptr(), logits.data_ptr(),
@@ -751,7 +888,22 @@ class UNetTrainEngine:
             self._replay("fwd", self.fwd_ops, x)
         else:
             self._run(self.fwd_ops, x=x)
+        if self.strict and not torch.cuda.is_current_stream_capturing():
+            # the pack's overflow count travels to the host behind the forward; overflowed() reads it without a synchronisation
+            if self._overflow_host is None:
+                self._overflow_host = torch.zeros(1, dtype=torch.int32, pin_memory=True)
+                self._overflow_event = torch.cuda.Event()
+            self._overflow_host.copy_(self.overflow, non_blocking=True)
+            self._overflow_event.record()
         return self.logits
+
+    def overflowed(self):
+        """strict precision: True once a finished forward has counted packed weights past their layer's exponent (the weights grew
+        beyond the headroom fixed when the plan was built; that step's gradients are not finite). Never synchronises: the answer
+        trails the stream by the forwards that have not completed yet. The owner then builds a new plan (fresh exponents)."""
+        if not self.strict or self._overflow_event is None or not self._overflow_event.query():
+            return False
+        return int(self._overflow_host[0]) > 0
 
     def accumulate_into(self, targets):
         """targets: {parameter name: fp32 contiguous .grad tensor}. Adds this step's gradients into them with ONE kernel

@@ -104,7 +104,9 @@ class UNet(nn.Module):
         self._engines = {}
         self._engines_version = None
         self._train_engines = {}
-        self.precision = None  # None: RSB_PRECISION or "strict" (see robosat_b200.engine.UNetEngine)
+        self.precision = None  # None: RSB_PRECISION or "strict" (see robosat_b200.engine.UNetEngine); eval plans only
+        # training plans: None = RSB_TRAIN_PRECISION or "fast"; "strict" = hi/lo fp16 forward (robosat_b200.train_engine.UNetTrainEngine)
+        self.train_precision = None
         # loss.backward() adds into existing .grad tensors with one kernel instead of one autograd add per parameter
         # (False: hand every gradient to autograd, e.g. when tensor hooks on parameters must fire)
         self.fused_grad_accumulation = True
@@ -134,16 +136,23 @@ class UNet(nn.Module):
         return super().train(mode)
 
     def _train_engine_for(self, x):
-        from robosat_b200.train_engine import UNetTrainEngine
+        from robosat_b200.train_engine import UNetTrainEngine, default_train_precision
 
-        key = (tuple(x.shape), x.dtype, x.device.index)
+        precision = self.train_precision or default_train_precision()
+        key = (tuple(x.shape), x.dtype, x.device.index, precision)
         eng = self._train_engines.get(key)
+        if eng is not None and eng.overflowed():
+            # strict plan: the weights outgrew the exponents fixed when it was built (that step's gradients were not finite and
+            # the guarded optimiser step skipped it); a new plan takes fresh exponents from the current weights
+            eng = None
+            del self._train_engines[key]
         if eng is None:
             # live references: the plan reads the current storage of every parameter / buffer at each step
             params = dict(self.named_parameters())
             params.update(dict(self.named_buffers()))
             h, w = (x.shape[2], x.shape[3]) if x.dtype == torch.float32 else (x.shape[1], x.shape[2])
-            eng = UNetTrainEngine(params, self.num_classes, x.shape[0], h, w, device=x.device, loss_scale=self.loss_scale)
+            eng = UNetTrainEngine(params, self.num_classes, x.shape[0], h, w, device=x.device, loss_scale=self.loss_scale,
+                                  precision=precision)
             self._train_engines[key] = eng
         return eng
 

@@ -1,7 +1,9 @@
 """Training-step throughput (BASELINE.json configs[2]: ResNet50-UNet, 2 classes, Lovasz loss, 3x512x512, batch 16, 1 GPU).
 One step = zero_grad + forward (train-mode BN) + Lovasz loss + backward + Adam, through the public module API.
 
-    python scripts/bench_train.py [--batch 16 --size 512 --steps 10 --warmup 3]
+    python scripts/bench_train.py [--batch 16 --size 512 --steps 10 --warmup 3 --precision fast|strict]
+
+--precision sets UNet.train_precision (fast: single fp16 forward; strict: hi/lo fp16 forward, robosat_b200/train_engine.py).
 """
 import argparse
 import json
@@ -23,10 +25,12 @@ def main():
     ap.add_argument("--size", type=int, default=512)
     ap.add_argument("--steps", type=int, default=10)
     ap.add_argument("--warmup", type=int, default=3)
+    ap.add_argument("--precision", choices=("fast", "strict"), default="fast")
     args = ap.parse_args()
     dev = torch.device("cuda:0")
     net = torch.nn.DataParallel(UNet(2, pretrained=False), device_ids=[0]).to(dev)
     net.load_state_dict(synth.make_state_dict(2, seed=0))
+    net.module.train_precision = args.precision
     opt = Adam(net.parameters(), lr=1e-4)
     opt.mark_used([not n.startswith("module.resnet.fc.") for n, _ in net.named_parameters()])
     crit = LovaszLoss2d().to(dev)
@@ -67,9 +71,10 @@ def main():
     for i in range(3):
         step(i, True)
     out = {"metric": "512x512 tiles/sec (train fwd+bwd+Lovasz+Adam)", "value": args.batch * args.steps / (total / 1e3), "unit": "tiles/s",
-           "ms_per_step": total / args.steps, "batch": args.batch, "size": args.size, "steps": args.steps,
+           "precision": args.precision, "ms_per_step": total / args.steps, "batch": args.batch, "size": args.size, "steps": args.steps,
            "breakdown_ms": {k: sum(v) / len(v) for k, v in ev.items()}, "loss_first": float(losses[0]), "loss_last": float(losses[-1]),
-           "fwd_bwd_dense_tflops": args.batch * args.steps * 500.246 / (total / 1e3) / 1e3}
+           "fwd_bwd_dense_tflops": args.batch * args.steps * 500.246 / (total / 1e3) / 1e3,
+           "gpu": torch.cuda.get_device_name(dev)}
     print(json.dumps(out))
 
 
